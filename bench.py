@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — ops merged/sec of the Peritext op-log apply + flatten hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c4|c2|c3|c5] [--docs D] [--impl engine|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c4|c2|c3|c5] [--docs D] [--impl engine|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" is one pass of the hot path (pt_batch_merge: apply every op of every log + flatten to spans + digest) over one
@@ -173,8 +173,10 @@ def run_reference(args, rank, world):
         replay_packed(batch, threads=cores)
     per_step = []
     for _ in range(args.steps):
-        _, dt = replay_packed(batch, threads=cores)
+        merged, dt = replay_packed(batch, threads=cores)
         per_step.append(dt)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, merged, DUMP_BYTES)
     ms = 1e3 * sum(per_step) / max(1, args.steps)
     value = batch.n_ops / (ms / 1e3)
     med = sorted(per_step)[len(per_step) // 2]
@@ -306,6 +308,52 @@ class DeviceRun:
         self.eng.close()
 
 
+DUMP_BYTES = 64_000_000   # --dump-outputs writes at most this much (split evenly over the ranks)
+DUMP_SEED = 0x5EED
+
+
+def _ranges(starts, counts):
+    """Concatenation of range(s, s + c) over the pairs: the element indices of variable-length records."""
+    starts, counts = np.asarray(starts, np.int64), np.asarray(counts, np.int64)
+    first = np.concatenate([[0], np.cumsum(counts)[:-1]])
+    return np.arange(int(counts.sum()), dtype=np.int64) + np.repeat(starts - first, counts)
+
+
+def dump_outputs(out_dir, merged, budget, prefix=""):
+    """Writes a MergedBatch (what pt_batch_download hands the caller) as float64 .npy files, at most `budget` bytes, so
+    that two builds can be compared array for array.  Every field is a u32, exact in float64; each 64-bit digest word is
+    stored as its low and high halves.  Logs are chosen in one fixed seeded order, so equal outputs give equal files.
+      results.npy          [n, 9] log, status, n_elems, n_visible, n_spans, digest[0] lo, hi, digest[1] lo, hi
+                           (every log if that takes at most half the budget, else a sample)
+      sample_logs.npy      [k, 4] log, n_visible, n_spans, comments: the logs whose full output follows, as many as fit
+      sample_tokens.npy    their visible tokens, log after log
+      sample_spans.npy     [m, 3] start, flags, link_attr of their spans (flags >> 8 = the span's comment count)
+      sample_comments.npy  the comment ranks of those spans, span after span (offset-free, unlike comment_off)"""
+    res = merged.results
+    n = len(res)
+    order = np.random.default_rng(DUMP_SEED).permutation(n)
+    rows = np.sort(order[: min(n, budget // 2 // (9 * 8))])
+    dg = res["digest"][rows]
+    results = np.stack([np.asarray(c, np.float64) for c in (rows, res["status"][rows], res["n_elems"][rows], res["n_visible"][rows],
+                        res["n_spans"][rows], dg[:, 0] & 0xFFFFFFFF, dg[:, 0] >> 32, dg[:, 1] & 0xFFFFFFFF, dg[:, 1] >> 32)], axis=1)
+    span_off, n_spans = merged.span_off[:n].astype(np.int64), res["n_spans"].astype(np.int64)
+    per_span = np.concatenate([[0], np.cumsum(merged.spans["flags"] >> 8, dtype=np.int64)])
+    n_comments = per_span[span_off + n_spans] - per_span[span_off]
+    cost = 8 * (4 + res["n_visible"].astype(np.int64) + 3 * n_spans + n_comments)
+    room = budget - results.nbytes - 5 * 256             # the .npy header of each file
+    sel = np.sort(order[: int(np.searchsorted(np.cumsum(cost[order]), room, side="right"))])
+    spans = merged.spans[_ranges(span_off[sel], n_spans[sel])]
+    arrays = {"results": results,
+              "sample_logs": np.stack([sel, res["n_visible"][sel], n_spans[sel], n_comments[sel]], axis=1),
+              "sample_tokens": merged.text[_ranges(merged.text_off[sel], res["n_visible"][sel])],
+              "sample_spans": np.stack([spans["start"], spans["flags"], spans["link_attr"]], axis=1),
+              "sample_comments": merged.comment_pool[_ranges(spans["comment_off"], spans["flags"] >> 8)]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.asarray(a, np.float64))
+    return {name: a.shape[0] for name, a in arrays.items()}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -320,7 +368,10 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the extra configs (c2, c3) reported beside the headline")
     ap.add_argument("--no-weak", action="store_true", help="N > 1: skip the weak-scaling measurement")
     ap.add_argument("--e2e-compact", action="store_true", help="also time the e2e leg on the compact wire format (host conversion inside the timed region)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's outputs to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "engine" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -367,6 +418,8 @@ def main():
 
     run = DeviceRun(torch, dist, dev, local_rank, world, batch, counts)
     total_ms, per_step, launches = run.timed(args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, run.eng.download(), DUMP_BYTES // world, f"rank{rank}_" if world > 1 else "")
     lone_ms = run.lone_merge_ms(min(5, args.steps))
     results, ok, converged = run.check()
     stats = run.eng.stats()
